@@ -1,6 +1,6 @@
-"""Minimal stand-in for the pure-Python `trampoline` package (setup.py:46 of the reference), which is
-not installed in this image and cannot be downloaded.  Used ONLY by tests/golden/make_golden.py to
-import the reference here; semantics per its usage in torchsde/_brownian/brownian_interval.py:183-315:
+"""Minimal stand-in for the pure-Python `trampoline` package (setup.py:46 of the reference), which
+torch does not depend on and may not be installed.  Used only to import the reference: by the golden
+generators under tests/golden/ and next to the copy that oracle/stage_reference.py stages; semantics per its usage in torchsde/_brownian/brownian_interval.py:183-315:
 run a generator; a yielded generator is run and its return value sent back; `raise TailCall(g)`
 replaces the current frame by g."""
 class TailCall(Exception):

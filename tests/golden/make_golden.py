@@ -1,7 +1,7 @@
 """Generate the golden vectors under tests/golden/ by running the REFERENCE (google-research/
-torchsde v0.2.6, mounted read-only at /root/reference) in this container on the CPU.
+torchsde v0.2.6, a source tree named by TSDE_REFERENCE_SRC) on the CPU.
 
-    python tests/golden/make_golden.py
+    TSDE_REFERENCE_SRC=/path/to/torchsde-0.2.6 python tests/golden/make_golden.py
 
 The reference cannot travel to the GPU box, so its outputs are committed as small .npz fixtures
 together with this script.  `trampoline` (a pure-python dependency of the reference that is not
@@ -20,7 +20,10 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, os.path.join(ROOT, 'oracle', 'refshim'))
-sys.path.insert(0, '/root/reference')
+REFERENCE = os.environ.get('TSDE_REFERENCE_SRC')
+if not REFERENCE:
+    sys.exit("make_golden.py: set TSDE_REFERENCE_SRC to a torchsde v0.2.6 source tree (the directory holding torchsde/)")
+sys.path.insert(0, REFERENCE)
 sys.path.insert(0, ROOT)
 
 import numpy as np  # noqa: E402
@@ -125,9 +128,8 @@ def ito_diagonal_fixture():
     reference's own NeuralDiagonal(d=5), seeds as diagnostics/utils.py:123-127."""
     import random
     from tests import problems as my_problems
-    sys.path.insert(0, '/root/reference')
     import importlib.util
-    spec = importlib.util.spec_from_file_location('ref_problems', '/root/reference/tests/problems.py')
+    spec = importlib.util.spec_from_file_location('ref_problems', os.path.join(REFERENCE, 'tests', 'problems.py'))
     ref_problems = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(ref_problems)
     torch.set_default_dtype(torch.float64)

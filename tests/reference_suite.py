@@ -3,8 +3,9 @@
 
     python tests/reference_suite.py [extra pytest args]        # on a CUDA box
 
-`__graft_entry__.build()` stages the reference's tests/ under the git-ignored baseline/_ref_tests/reference_tests (they
-cannot be committed: reference sources).  This runner puts an import alias `torchsde -> torchsde_b200`
+`__graft_entry__.build()` stages the reference's tests/ under the git-ignored oracle/_ref/tests/reference_tests where
+TSDE_REFERENCE_SRC names a reference source tree (oracle/stage_reference.py; they cannot be committed: reference
+sources).  This runner puts an import alias `torchsde -> torchsde_b200`
 (tests/as_torchsde) first on sys.path and runs them.  The reference parametrises most tests over ['cpu', 'cuda'];
 this package has no CPU path by design, so the CPU parametrisations are deselected and only counted; tests without a
 `device` parameter get the GPU as torch's default device (tests/as_torchsde/refsuite_plugin.py).  Output: the
@@ -18,17 +19,15 @@ import sys
 import time
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-SUITE = os.path.join(ROOT, 'baseline', '_ref_tests', 'reference_tests')
+sys.path.insert(0, ROOT)
+from oracle.stage_reference import TESTS as SUITE  # noqa: E402
 ALIAS = os.path.join(ROOT, 'tests', 'as_torchsde')
 
 
 def main():
     if not os.path.isdir(SUITE):
-        sys.path.insert(0, ROOT)
-        import __graft_entry__ as g
-        g.stage_reference()
-    if not os.path.isdir(SUITE):
-        print(json.dumps({"unavailable": "baseline/_ref_tests/reference_tests is absent (run build() where /root/reference is mounted)"}))
+        print(json.dumps({"unavailable": "oracle/_ref/tests/reference_tests is absent (run build() with TSDE_REFERENCE_SRC "
+                                         "naming a torchsde v0.2.6 source tree)"}))
         return 0
     env = dict(os.environ, PYTHONPATH=os.pathsep.join([ALIAS, ROOT]))
     # CPU parametrisations: ids contain 'cpu' or 'device0' (devices = [cpu, gpu] lists)

@@ -253,9 +253,9 @@ def test_bench_reference_arm_prints_one_contract_line():
         assert key in d, key
     assert d['value'] > 0 and d['e2e']['value'] == d['value'] and d['e2e']['h2d_bytes_per_step'] == 0
     cb = d['cpu_baseline']
-    # the reference itself where build() has staged it under baseline/_ref (git-ignored, travels with the snapshot);
-    # the numpy port only where that directory is absent
-    staged = os.path.isdir(os.path.join(ROOT, 'baseline', '_ref', 'torchsde'))
+    # the reference itself where build() has staged it under oracle/_ref (git-ignored, travels with a copy of the
+    # working tree); the numpy port only where that directory is absent
+    staged = os.path.isdir(os.path.join(ROOT, 'oracle', '_ref', 'pkg', 'torchsde'))
     assert cb['kind'] == ('reference' if staged else 'port') and cb['cores'] >= 1
     assert d['config']['workload'] == 'cfg2' and d['config']['method'] == 'milstein' 
 
